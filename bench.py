@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- headline benchmark of the B200 VP8 decode hot path.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload 1080p|features|4k|720p]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload 1080p|features|4k|720p] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): "1080p30 IVF decode, 1 GPU".  No >= 1080p VP8 material exists, so the
 streams are synthetic: six DISTINCT 30-frame GOPs produced by the reference's own encoder from seeded
@@ -373,7 +373,12 @@ def main():
     ap.add_argument("--ncu-summary", default=os.path.join(ROOT, "profiles", "r2_final_ncu_full_summary.csv"),
                     help="condensed `ncu --set full` capture; it was taken with 64 streams per launch (--ncu-streams)")
     ap.add_argument("--ncu-streams", type=int, default=64)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the frames the last e2e step decoded to DIR/*.npy (a seeded sample of "
+                         "whole frames and per-plane sums of every frame), so that two builds can be compared")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     a.warmup = max(a.warmup, 0)
 
     from alfalfa_b200 import multigpu as M
@@ -615,6 +620,8 @@ def main():
     # sanity: the output buffer holds pictures (the real 720p vector opens with a flat frame: look at a few)
     probe = np.frombuffer(C.string_at(dst, min(int(out_bytes), 8 * ctx2_display_bytes)), dtype=np.uint8)
     assert probe.std() > 1.0
+    if a.dump_outputs and rank == 0:
+        dump_decoded_frames(a.dump_outputs, dst, ctx2_display_bytes, w, h, nd.value, ns.value)
 
     # ---------------- one stream alone (latency-bound): a single instance, one worker, frames copied out ----------------
     one = make_ivf(w, h, instances[0])
@@ -705,6 +712,25 @@ def main():
             "exchange": exchange, "clocks": clocks}))
     if dist is not None:
         dist.destroy_process_group()
+
+
+def dump_decoded_frames(out_dir, dst, frame_bytes, w, h, n_decoded, n_shown, max_bytes=48 << 20):
+    """What the last timed e2e step handed its caller: the display rectangles (Y, U, V) of the shown frames in stream
+    order.  Written as float64 per-plane sums of every frame (frame_plane_sums.npy, [n_shown, 3]), a seeded sample of
+    whole frames (sampled_frames.npy, float32 [k, frame_bytes], at most `max_bytes`), their stream positions
+    (sampled_frame_index.npy) and [n_decoded, n_shown] (frame_counts.npy)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    frames = np.frombuffer((C.c_uint8 * (n_shown * frame_bytes)).from_address(dst.value), np.uint8).reshape(n_shown, frame_bytes)
+    ys, cs = w * h, ((w + 1) // 2) * ((h + 1) // 2)
+    planes = (frames[:, :ys], frames[:, ys:ys + cs], frames[:, ys + cs:])
+    sums = np.stack([p.sum(axis=1, dtype=np.float64) for p in planes], axis=1)
+    k = max(1, min(n_shown, max_bytes // (4 * frame_bytes)))
+    index = np.sort(np.random.default_rng(0).choice(n_shown, k, replace=False))
+    np.save(os.path.join(out_dir, "frame_plane_sums.npy"), sums)
+    np.save(os.path.join(out_dir, "sampled_frames.npy"), frames[index].astype(np.float32))
+    np.save(os.path.join(out_dir, "sampled_frame_index.npy"), index.astype(np.float64))
+    np.save(os.path.join(out_dir, "frame_counts.npy"), np.array([n_decoded, n_shown], np.float64))
 
 
 def ctx_bytes(w, h):

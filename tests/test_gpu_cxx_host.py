@@ -81,8 +81,7 @@ def test_cxx_reencode_equals_the_reference(tmp_path_factory, tmp_path, extra_fra
     import numpy as np
     import oracle_lib as O
     import test_gpu_reencode as R
-    if not (os.path.exists(R.REF_REENCODE) and os.path.exists(R.REF_DUMP)):
-        pytest.skip("oracle/_ref tools not built")
+    from reference_outputs import digests
     exe = _build(tmp_path_factory, "reencode_chunk")
     w, h, n = 176, 144, 4
     targets, pred, state = R.make_case(w, h, n, qi_a=36, qi_b=60)
@@ -98,4 +97,4 @@ def test_cxx_reencode_equals_the_reference(tmp_path_factory, tmp_path, extra_fra
                        stderr=subprocess.PIPE, timeout=600)
     assert r.returncode == 0 and r.stdout.decode().startswith("ok"), r.stderr.decode()[-500:]
     _, _, got = O.read_ivf(open(out, "rb").read())
-    assert got == want
+    assert digests(got) == want

@@ -9,7 +9,6 @@
    the emitted frames (CPU oracle, the unmodified reference decoder, this library's decoder) reconstructs
    exactly the raster the encoder kept as its LAST reference.
  * Encoder value semantics (copy, from a Decoder, export_decoder)."""
-import hashlib
 import os
 import subprocess
 import tempfile
@@ -18,6 +17,7 @@ import numpy as np
 import pytest
 
 import oracle_lib as O
+import reference_outputs as R
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -39,12 +39,13 @@ def synth(w, h, t, seed=7):
     return tuple(np.clip(a, 0, 255).astype(np.uint8) for a in (y, u, v))
 
 
-REF_ENCODE = os.path.join(ROOT, "oracle", "_ref", "ref_encode")
-needs_ref = pytest.mark.skipif(not os.path.exists(REF_ENCODE), reason="oracle/_ref/ref_encode not built")
-
-
-def reference_encode(frames, w, h, qi=None, target=None):
-    """the unmodified reference encoder on raw frames: list of compressed frames"""
+def reference_encode(frames, w, h, qi=None, target=None, two_pass=False):
+    """the unmodified reference encoder on raw frames: list of compressed frames.  Where oracle/_ref/ref_encode is not
+    built, this library's encoder codes them and every frame must have the digest stored for the reference's."""
+    k = R.key("ref_encode", w, h, qi, target, two_pass, frames)
+    tool = R.tool("ref_encode")
+    if tool is None:
+        return _product_encode_as_reference(k, frames, w, h, qi, target, two_pass)
     with tempfile.TemporaryDirectory() as d:
         raw, out = os.path.join(d, "src.yuv"), os.path.join(d, "o.ivf")
         with open(raw, "wb") as f:
@@ -54,10 +55,31 @@ def reference_encode(frames, w, h, qi=None, target=None):
         env = dict(os.environ, REF_RAW=raw)
         if target is not None:
             env["REF_TARGET"] = str(target)
-        r = subprocess.run([REF_ENCODE, out, str(w), str(h), str(len(frames)), "100000", str(qi or 0)], env=env,
+        if two_pass:
+            env["REF_TWO_PASS"] = "1"
+        r = subprocess.run([tool, out, str(w), str(h), str(len(frames)), "100000", str(qi or 0)], env=env,
                            capture_output=True, text=True)
         assert r.returncode == 0, r.stderr[-400:]
         _, _, chunks = O.read_ivf(open(out, "rb").read())
+    return R.check(k, chunks)
+
+
+def _product_encode_as_reference(k, frames, w, h, qi, target, two_pass):
+    from alfalfa_b200 import Context, Encoder
+    want = R.stored(k)
+    ctx = Context(w, h, max_frames=32)
+    enc = Encoder(ctx)
+    if two_pass:
+        enc.set_two_pass(True)
+    chunks = []
+    for t, planes in enumerate(frames):
+        blob = enc.encode_with_target_size(*planes, target)[0] if target is not None else enc.encode_with_quantizer(*planes, qi)
+        assert R.digest(blob) == want[t], "frame %d: %d bytes vs %d bytes of the reference encoder (digest differs)" % (
+            t, len(blob), want[t][0])
+        chunks.append(blob)
+    assert len(chunks) == len(want)
+    del enc
+    ctx.close()
     return chunks
 
 
@@ -89,7 +111,6 @@ def assert_same_decisions(pa, pb, what):
     assert bad.size == 0, "%s: coefficients differ at macroblocks %s" % (what, bad[:8])
 
 
-@needs_ref
 @pytest.mark.parametrize("size,n,qi", [((320, 240), 8, 40), ((176, 144), 6, 12), ((640, 368), 6, 70), ((1920, 1080), 3, 90)])
 def test_decisions_equal_the_reference_encoder(size, n, qi):
     from alfalfa_b200 import Context, Decoder, Encoder
@@ -115,7 +136,6 @@ def test_decisions_equal_the_reference_encoder(size, n, qi):
     ctx.close()
 
 
-@needs_ref
 def test_rd_parity_at_target_size_1080p():
     """SURVEY 8d config 3: encode_with_target_size at 20 000 and 60 000 bytes per frame over 30 raw 1080p
     frames next to the reference encoder: bytes within 5 %, SSIM >= reference - 0.005 (xc-enc-ssim.test:23),
@@ -176,7 +196,6 @@ def test_rd_parity_at_target_size_1080p():
     ctx.close()
 
 
-@needs_ref
 def test_first_inter_frame_estimates_price_vectors_at_zero():
     """The reference fills its motion-vector cost tables at the start of the first FULL inter-frame pass
     (encode_inter.cc:601-602), so the size estimates of the first inter frame price every vector at 0 and the
@@ -239,6 +258,18 @@ def test_encoder_value_semantics():
     ctx.close()
 
 
+def reference_decode_shown(ivf):
+    """digest of what the unmodified reference decoder shows for an IVF stream (ref_dump shown)"""
+    def run():
+        with tempfile.NamedTemporaryFile(suffix=".ivf") as f:
+            f.write(ivf)
+            f.flush()
+            r = subprocess.run([R.tool("ref_dump"), "shown", f.name], capture_output=True)
+        assert r.returncode == 0, r.stderr[-400:]
+        return [r.stdout]
+    return R.expected(R.key("ref_dump shown", ivf), run if R.tool("ref_dump") else None)[0]
+
+
 def psnr(a, b):
     mse = np.mean((a.astype(np.float64) - b.astype(np.float64)) ** 2)
     return 99.0 if mse == 0 else 10 * np.log10(255.0 ** 2 / mse)
@@ -272,13 +303,8 @@ def test_closed_loop_against_oracle_reference_and_own_decoder(size):
         mine.release()
     # motion-compensated frames (coarser quantiser, mostly noise left to code) stay below the key frame
     assert sum(len(f) for f in frames[1:]) / 5 < len(frames[0])
-    ref_dump = os.path.join(ROOT, "oracle", "_ref", "ref_dump")
-    if os.path.exists(ref_dump):  # the unmodified reference decoder agrees as well
-        with tempfile.NamedTemporaryFile(suffix=".ivf") as f:
-            f.write(write_ivf(w, h, frames))
-            f.flush()
-            raw = subprocess.run([ref_dump, "shown", f.name], capture_output=True).stdout
-        assert hashlib.sha1(raw).hexdigest() == hashlib.sha1(b"".join(recon_display)).hexdigest()
+    # the unmodified reference decoder agrees as well
+    assert R.digest(b"".join(recon_display)) == reference_decode_shown(write_ivf(w, h, frames))
     del enc, dec
     ctx.close()
 
@@ -448,7 +474,6 @@ def _noisy(w, h, t, amp):
     return tuple(np.clip(p.astype(np.int32) + rng.integers(-amp, amp + 1, p.shape), 0, 255).astype(np.uint8) for p in (y, u, v))
 
 
-@needs_ref
 @pytest.mark.parametrize("w,h,qi,amp,n", [(64, 64, 40, 20, 2), (176, 144, 70, 40, 2), (175, 143, 60, 35, 3), (320, 240, 110, 60, 2),
                                         (640, 368, 40, 30, 2)])
 def test_two_pass_key_frames_equal_the_reference_encoder(w, h, qi, amp, n):
@@ -458,11 +483,7 @@ def test_two_pass_key_frames_equal_the_reference_encoder(w, h, qi, amp, n):
     unmodified reference's (REF_TWO_PASS), noisy sources so that the trellis has something to decide"""
     from alfalfa_b200 import Context, Decoder, Encoder
     frames = [_noisy(w, h, t, amp) for t in range(n)]
-    os.environ["REF_TWO_PASS"] = "1"
-    try:
-        want = reference_encode(frames, w, h, qi=qi)
-    finally:
-        del os.environ["REF_TWO_PASS"]
+    want = reference_encode(frames, w, h, qi=qi, two_pass=True)
     one_pass = reference_encode(frames[:1], w, h, qi=qi)
     ctx = Context(w, h, max_frames=16)
     enc = Encoder(ctx)

@@ -16,12 +16,10 @@ import numpy as np
 import pytest
 
 import oracle_lib as O
+import reference_outputs as R
 from test_gpu_encoder import ROOT, reference_encode, synth
 
 pytestmark = pytest.mark.gpu
-REF_REENCODE = os.path.join(ROOT, "oracle", "_ref", "ref_reencode")
-REF_DUMP = os.path.join(ROOT, "oracle", "_ref", "ref_dump")
-needs_ref = pytest.mark.skipif(not (os.path.exists(REF_REENCODE) and os.path.exists(REF_DUMP)), reason="oracle/_ref tools not built")
 EMULATED = bool(os.environ.get("VP8GPU_SIMT_EMULATED"))
 SIZES = [(176, 144)] if EMULATED else [(176, 144), (640, 360)]
 
@@ -32,30 +30,46 @@ def ivf_bytes(w, h, chunks):
 
 
 def reference_reencode(w, h, targets, pred_chunks, state_blob, kf_q_weight, extra_frame_chunk):
-    """oracle/_ref/ref_reencode: the reference's Encoder::reencode; returns the emitted frames"""
-    with tempfile.TemporaryDirectory() as d:
-        raw, pred, state, out = (os.path.join(d, n) for n in ("t.yuv", "p.ivf", "s.bin", "o.ivf"))
-        with open(raw, "wb") as f:
-            for planes in targets:
-                for p in planes:
-                    f.write(np.ascontiguousarray(p).tobytes())
-        open(pred, "wb").write(ivf_bytes(w, h, pred_chunks))
-        open(state, "wb").write(state_blob)
-        r = subprocess.run([REF_REENCODE, out, str(w), str(h), raw, pred, state, repr(kf_q_weight), str(int(extra_frame_chunk))],
-                           capture_output=True, text=True)
-        assert r.returncode == 0, r.stderr[-400:]
-        _, _, chunks = O.read_ivf(open(out, "rb").read())
-    return chunks
+    """oracle/_ref/ref_reencode: the reference's Encoder::reencode; returns the digests (reference_outputs.digest) of
+    the emitted frames"""
+    def run():
+        with tempfile.TemporaryDirectory() as d:
+            raw, pred, state, out = (os.path.join(d, n) for n in ("t.yuv", "p.ivf", "s.bin", "o.ivf"))
+            with open(raw, "wb") as f:
+                for planes in targets:
+                    for p in planes:
+                        f.write(np.ascontiguousarray(p).tobytes())
+            open(pred, "wb").write(ivf_bytes(w, h, pred_chunks))
+            open(state, "wb").write(state_blob)
+            r = subprocess.run([R.tool("ref_reencode"), out, str(w), str(h), raw, pred, state, repr(kf_q_weight),
+                                str(int(extra_frame_chunk))], capture_output=True, text=True)
+            assert r.returncode == 0, r.stderr[-400:]
+            return O.read_ivf(open(out, "rb").read())[2]
+    k = R.key("ref_reencode", w, h, targets, pred_chunks, state_blob, kf_q_weight, bool(extra_frame_chunk))
+    return R.expected(k, run if R.tool("ref_reencode") else None)
 
 
 def reference_state_after(w, h, chunks, n):
-    """Decoder::serialize of the reference decoder after n frames (ref_dump state)"""
+    """Decoder::serialize of the reference decoder after n frames (ref_dump state).  Where the reference is not built,
+    this library's Decoder::serialize, which must have the digest stored for the reference's blob."""
+    k = R.key("ref_dump state", w, h, chunks[:n])
+    if R.tool("ref_dump") is None:
+        from alfalfa_b200 import Context, Decoder
+        ctx = Context(w, h, max_frames=16)
+        dec = Decoder(ctx)
+        for c in chunks[:n]:
+            dec.get_frame_output(c)[1].release()
+        blob = dec.serialize()
+        del dec
+        ctx.close()
+        assert R.digest(blob) == R.stored(k)[0], "Decoder::serialize differs from the reference's blob"
+        return blob
     with tempfile.TemporaryDirectory() as d:
         path = os.path.join(d, "a.ivf")
         open(path, "wb").write(ivf_bytes(w, h, chunks))
-        r = subprocess.run([REF_DUMP, "state", path, str(n)], capture_output=True)
+        r = subprocess.run([R.tool("ref_dump"), "state", path, str(n)], capture_output=True)
         assert r.returncode == 0, r.stderr[-400:]
-        return r.stdout
+        return R.check(k, [r.stdout])[0]
 
 
 def make_case(w, h, n, qi_a, qi_b):
@@ -84,7 +98,6 @@ def product_reencode(w, h, targets, pred_chunks, state_blob, kf_q_weight, extra_
     return out["frames"], out["in_step"]
 
 
-@needs_ref
 def test_whole_chunk_the_same_with_the_shortcuts_off():
     """VP8GPU_ENC_SPECULATE=0: the loop-filter trials one by one and the decode of every written frame through the
     full parse instead of the token lists it was written from -- the same bytes, the receiver still in step"""
@@ -93,10 +106,9 @@ def test_whole_chunk_the_same_with_the_shortcuts_off():
     targets, pred, state = make_case(w, h, n, qi_a=40, qi_b=64)
     want = reference_reencode(w, h, targets, pred, state, 0.75, False)
     got, in_step = product_reencode(w, h, targets, pred, state, 0.75, False, env={"VP8GPU_ENC_SPECULATE": "0"})
-    assert got == want and in_step
+    assert R.digests(got) == want and in_step
 
 
-@needs_ref
 @pytest.mark.parametrize("size", SIZES)
 @pytest.mark.parametrize("kf_q_weight", [1.0, 0.75])
 def test_extra_frame_chunk_is_reencoded_byte_for_byte_like_the_reference(size, kf_q_weight):
@@ -109,14 +121,12 @@ def test_extra_frame_chunk_is_reencoded_byte_for_byte_like_the_reference(size, k
     got, in_step = product_reencode(w, h, targets, pred, state, kf_q_weight, True)
     assert len(got) == len(want) == n - 1
     for i, (a, b) in enumerate(zip(got, want)):
-        assert a == b, "frame %d: %d vs %d bytes, first difference at %d" % (
-            i + 1, len(a), len(b), next((k for k in range(min(len(a), len(b))) if a[k] != b[k]), -1))
+        assert R.digest(a) == b, "frame %d: %d vs %d bytes" % (i + 1, len(a), b[0])
     # and the Encoder moved the way a receiver moves: a decoder resumed from the blob that decodes the emitted
     # frames ends up equal to export_decoder()
     assert in_step
 
 
-@needs_ref
 @pytest.mark.parametrize("size", SIZES)
 @pytest.mark.parametrize("kf_q_weight", [1.0, 0.5])
 def test_whole_chunk_is_reencoded_byte_for_byte_like_the_reference(size, kf_q_weight):
@@ -130,13 +140,11 @@ def test_whole_chunk_is_reencoded_byte_for_byte_like_the_reference(size, kf_q_we
     got, in_step = product_reencode(w, h, targets, pred, state, kf_q_weight, False)
     assert len(got) == len(want) == n
     for i, (a, b) in enumerate(zip(got, want)):
-        assert a == b, "frame %d: %d vs %d bytes, first difference at %d" % (
-            i, len(a), len(b), next((k for k in range(min(len(a), len(b))) if a[k] != b[k]), -1))
+        assert R.digest(a) == b, "frame %d: %d vs %d bytes" % (i, len(a), b[0])
     assert got[0][0] & 1, "the chunk no longer starts with a key frame"
     assert in_step
 
 
-@needs_ref
 def test_reencoded_frames_differ_from_the_prediction_frames_but_keep_their_modes():
     """the point of update_residues: same decisions, new residues (the references are another reconstruction)"""
     w, h, n = 176, 144, 3
@@ -213,7 +221,6 @@ def _full_name(prefix):
     return hits[0]
 
 
-@needs_ref
 @pytest.mark.parametrize("prev,this,nframes", VECTOR_CASES)
 def test_update_residues_on_libvpx_prediction_streams(prev, this, nframes):
     pw, ph, prev_chunks = _golden(_full_name(prev))
@@ -228,11 +235,10 @@ def test_update_residues_on_libvpx_prediction_streams(prev, this, nframes):
     got, in_step = product_reencode(w, h, targets, chunks, state, 0.75, True)
     assert len(got) == len(want) == len(chunks) - 1
     for i, (a, b) in enumerate(zip(got, want)):
-        assert a == b, "frame %d: %d vs %d bytes" % (i + 1, len(a), len(b))
+        assert R.digest(a) == b, "frame %d: %d vs %d bytes" % (i + 1, len(a), b[0])
     assert in_step
 
 
-@needs_ref
 @pytest.mark.parametrize("prev", ["07b5eb1e", "4fca93f3", "a4dace04", "ced8ea72", "d4e9f670", "df225756"])
 def test_whole_chunk_after_a_libvpx_stream(prev):
     """options 1 + 4 when the receiver's state comes from a libvpx stream: updated motion-vector and mode
@@ -246,4 +252,4 @@ def test_whole_chunk_after_a_libvpx_stream(prev):
     state = reference_state_after(w, h, prev_chunks, len(prev_chunks))
     want = reference_reencode(w, h, frames, pred, state, 0.75, False)
     got, in_step = product_reencode(w, h, frames, pred, state, 0.75, False)
-    assert got == want and in_step
+    assert R.digests(got) == want and in_step

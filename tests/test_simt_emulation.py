@@ -69,9 +69,7 @@ def test_stream_decode_and_device_token_decoder_emulated(simt_lib):
 
 def test_reencode_against_the_reference_emulated(simt_lib):
     """Encoder::reencode / update_residues (SURVEY 8 f3): k_reenc_inter / k_reenc_intra + the host orchestration,
-    byte for byte against oracle/_ref/ref_reencode on reference-encoder and libvpx prediction streams"""
-    if not os.path.exists(os.path.join(ROOT, "oracle", "_ref", "ref_reencode")):
-        pytest.skip("oracle/_ref/ref_reencode not built (make -C oracle ref)")
+    byte for byte against the reference's Encoder::reencode on reference-encoder and libvpx prediction streams"""
     run_gpu_tests_emulated(simt_lib, ["tests/test_gpu_reencode.py"])
 
 
@@ -94,8 +92,7 @@ def test_reverse_thread_order_gives_the_same_results(simt_lib):
     run_gpu_tests_emulated(simt_lib, ["tests/test_gpu_parity.py", "-k", "every_frame_matches_oracle or (fileplayer and not ff2941 and not 2a4c049c)"],
                            env_extra=rev)
     run_gpu_tests_emulated(simt_lib, ["tests/test_gpu_encoder.py", "-k", "decisions_equal and not size3"], env_extra=rev)
-    if os.path.exists(os.path.join(ROOT, "oracle", "_ref", "ref_reencode")):
-        run_gpu_tests_emulated(simt_lib, ["tests/test_gpu_reencode.py"], env_extra=rev)
+    run_gpu_tests_emulated(simt_lib, ["tests/test_gpu_reencode.py"], env_extra=rev)
 
 
 def test_no_misaligned_vector_access_in_the_kernels(simt_lib):
@@ -111,7 +108,6 @@ def test_no_misaligned_vector_access_in_the_kernels(simt_lib):
     assert r.returncode == 0 and os.path.exists(san), r.stderr[-2000:]
     args = ["tests/test_gpu_parity.py", "-k", "fileplayer and (0b546dad or a4dace04 or e01c6f92 or 8bf4c5bb)"]
     run_gpu_tests_emulated(san, args, env_extra={"LD_PRELOAD": ubsan})
-    if os.path.exists(os.path.join(ROOT, "oracle", "_ref", "ref_reencode")):
-        run_gpu_tests_emulated(san, ["tests/test_gpu_reencode.py"], env_extra={"LD_PRELOAD": ubsan})
+    run_gpu_tests_emulated(san, ["tests/test_gpu_reencode.py"], env_extra={"LD_PRELOAD": ubsan})
     # the encoder's predictor (packed filters on staged windows, word stores into the candidate buffers)
     run_gpu_tests_emulated(san, ["tests/test_gpu_encoder.py", "-k", "(decisions_equal and not size3) or two_pass"], env_extra={"LD_PRELOAD": ubsan})

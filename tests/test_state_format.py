@@ -8,7 +8,6 @@ GPU part: the whole Decoder blob (state + LAST raster) equals the reference's by
 deserialised from the REFERENCE's blob continues the stream bit-exactly, and the reference resumes from OUR blob
 (ref_dump resume) with the reference decode's output."""
 import ctypes as C
-import hashlib
 import os
 import subprocess
 import tempfile
@@ -16,17 +15,16 @@ import tempfile
 import pytest
 
 import oracle_lib as O
+import reference_outputs as R
 from alfalfa_b200 import capi
 from conftest import GOLDEN_DIR, golden_vectors
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-TOOL = os.path.join(ROOT, "oracle", "_ref", "ref_dump")
-needs_tool = pytest.mark.skipif(not os.path.exists(TOOL), reason="oracle/_ref/ref_dump not built (make -C oracle ref)")
 FEATURES = os.path.join(ROOT, "bench_data", "features1080p_12f.ivf")
 
 
 def _ref_blob(path, n):
-    return subprocess.run([TOOL, "state", path, str(n)], stdout=subprocess.PIPE, check=True).stdout
+    return subprocess.run([R.tool("ref_dump"), "state", path, str(n)], stdout=subprocess.PIPE, check=True).stdout
 
 
 def _state_record(blob):
@@ -34,6 +32,28 @@ def _state_record(blob):
     assert blob[5] == 4                                                                # DECODER_STATE
     n = int.from_bytes(blob[6:10], "little")
     return blob[5:5 + 5 + n]
+
+
+def _ref_state_record(path, n):
+    """digest of the DECODER_STATE record of the reference's Decoder::serialize after n frames of `path`"""
+    k = R.key("ref_dump state record", open(path, "rb").read(), n)
+    return R.expected(k, (lambda: [_state_record(_ref_blob(path, n))]) if R.tool("ref_dump") else None)[0]
+
+
+def _ref_blob_digest(path, n):
+    """digest of the reference's whole Decoder::serialize blob (state + LAST raster) after n frames of `path`"""
+    k = R.key("ref_dump state", open(path, "rb").read(), n)
+    return R.expected(k, (lambda: [_ref_blob(path, n)]) if R.tool("ref_dump") else None)[0]
+
+
+def _ref_resume_digest(blob, path, n):
+    """digest of what the reference shows after resuming from `blob` at frame n of `path` (ref_dump resume)"""
+    def run():
+        with tempfile.NamedTemporaryFile(suffix=".state") as tf:
+            tf.write(blob)
+            tf.flush()
+            return [subprocess.run([R.tool("ref_dump"), "resume", tf.name, path, str(n)], stdout=subprocess.PIPE, check=True).stdout]
+    return R.expected(R.key("ref_dump resume", blob, open(path, "rb").read(), n), run if R.tool("ref_dump") else None)[0]
 
 
 def _product_state_blob(path, n):
@@ -57,7 +77,6 @@ def _product_state_blob(path, n):
     return blob
 
 
-@needs_tool
 @pytest.mark.parametrize("name", golden_vectors())
 def test_state_record_equals_the_reference(name):
     path = os.path.join(GOLDEN_DIR, name)
@@ -65,15 +84,14 @@ def test_state_record_equals_the_reference(name):
     if frames[0][0] & 1:
         pytest.skip("vector does not start with a key frame")
     for n in sorted({1, min(len(frames), 7), min(len(frames), 29)}):
-        assert _product_state_blob(path, n) == _state_record(_ref_blob(path, n)), "after %d frames" % n
+        assert R.digest(_product_state_blob(path, n)) == _ref_state_record(path, n), "after %d frames" % n
 
 
-@needs_tool
 def test_state_record_on_the_feature_stream_with_segmentation_and_filter_deltas():
     kinds = set()
     for n in (1, 3, 5, 8, 12):
         ours = _product_state_blob(FEATURES, n)
-        assert ours == _state_record(_ref_blob(FEATURES, n))
+        assert R.digest(ours) == _ref_state_record(FEATURES, n)
         body = ours[9 + 5 + 1101:]
         kinds.add((body[0], ours[-14] if body[0] == 6 else None))
     assert any(k[0] == 6 for k in kinds), "no position with segmentation enabled was covered"
@@ -90,7 +108,6 @@ def test_state_deserialize_rejects_garbage():
     assert L.vp8gpu_state_deserialize(bytes(bad[:9]) + b"\x07" + bytes(bad[10:]), len(bad), C.byref(st)) != 0
 
 
-@needs_tool
 @pytest.mark.gpu
 @pytest.mark.parametrize("path,n", [(os.path.join(GOLDEN_DIR, "0b546dad90ddefea5085c7751b5fa2f117630b1c"), 9),
                                      (os.path.join(GOLDEN_DIR, "2a4c049c2f8e3a19ee39ffd7074cecd68006a101"), 20)])
@@ -106,17 +123,15 @@ def test_decoder_blob_equals_the_reference_and_both_sides_resume_from_it(path, n
         r.release()
     size = C.c_size_t(0)
     assert L.vp8gpu_decoder_serialize(dec.h, None, 0, C.byref(size)) == capi.ERR_NOMEM
-    ours, theirs = dec.serialize(), _ref_blob(path, n)
+    ours = dec.serialize()
     assert len(ours) == size.value
     # golden / alternative are not part of the format: the reference blob only carries LAST as well
-    assert ours == theirs
+    assert R.digest(ours) == _ref_blob_digest(path, n)
+    theirs = _ref_blob(path, n) if R.tool("ref_dump") else ours  # (byte-equal, by the digest above)
     # (a) the product resumes from the REFERENCE's blob
     resumed = Decoder.deserialize(ctx, theirs)
     # the truth for "resume with golden = alternative = last": the reference itself, from its own blob
-    with tempfile.NamedTemporaryFile(suffix=".state") as tf:
-        tf.write(ours)
-        tf.flush()
-        want = subprocess.run([TOOL, "resume", tf.name, path, str(n)], stdout=subprocess.PIPE, check=True).stdout
+    want = _ref_resume_digest(ours, path, n)
     got = b""
     for f in frames[n:]:
         shown, r = resumed.get_frame_output(f)
@@ -124,6 +139,6 @@ def test_decoder_blob_equals_the_reference_and_both_sides_resume_from_it(path, n
             got += r.display_bytes()
         r.release()
     # (b) ... and that run of the reference read OUR blob: both continuations agree
-    assert hashlib.sha1(got).hexdigest() == hashlib.sha1(want).hexdigest() and len(got) == len(want)
+    assert R.digest(got) == want
     del dec, resumed
     ctx.close()
