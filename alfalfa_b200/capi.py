@@ -79,6 +79,7 @@ MB_DTYPE = np.dtype([("tok_off", "<u4"), ("tok_cnt", "<u2"), ("y_mode", "u1"), (
                      ("b_modes", "<u8")])
 
 OPT_DEVICE_TOKENS = 1  # VP8GPU_OPT_DEVICE_TOKENS
+QUALITY_BEST, QUALITY_REALTIME = 0, 1  # VP8GPU_QUALITY_* (EncoderQuality, encoder.hh:56-60)
 
 # every symbol include/vp8gpu.h declares: name -> (restype, argtypes)
 _vp = C.c_void_p
@@ -147,6 +148,7 @@ SYMBOLS = {
     "vp8gpu_encoder_export_decoder": (C.c_int, [_vp, _pp]),
     "vp8gpu_encoder_minihash": (C.c_int, [_vp, C.POINTER(C.c_uint32)]),
     "vp8gpu_encoder_set_two_pass": (C.c_int, [_vp, C.c_int]),
+    "vp8gpu_encoder_set_quality": (C.c_int, [_vp, C.c_int]),
     "vp8gpu_encoder_update_residues": (C.c_int, [_vp, _u8p, C.c_size_t, _u8p, _u8p, C.c_size_t, _vp, C.c_int, C.c_int,
                                                  _u8p, C.c_size_t, C.POINTER(C.c_size_t)]),
     "vp8gpu_encoder_reencode_as_interframe": (C.c_int, [_vp, _u8p, C.c_size_t, _u8p, _u8p, C.c_size_t, _vp, C.c_int,

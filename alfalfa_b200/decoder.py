@@ -393,9 +393,10 @@ def decode_ivf(ctx, ivf_bytes, threads=1, want_output=True):
 
 class Encoder:
     """Encoder (encoder/encoder.hh:345-382): a copyable value like the reference's.  Source frames are
-    display-size (Y, U, V) numpy planes; the result is one compressed VP8 frame."""
+    display-size (Y, U, V) numpy planes; the result is one compressed VP8 frame.  quality: "realtime" (Salsify's
+    setting, the default) or "best" (ExCamera's xc-enc default), see set_quality."""
 
-    def __init__(self, ctx, _h=None):
+    def __init__(self, ctx, _h=None, quality="realtime"):
         self.ctx, self.L = ctx, ctx.L
         self.h = C.c_void_p()
         if _h is not None:
@@ -403,6 +404,8 @@ class Encoder:
         else:
             check(self.L.vp8gpu_encoder_create(ctx.h, C.byref(self.h)), ctx.h, "encoder_create")
         self._out = np.empty(ctx.width * ctx.height * 3 + (1 << 16), np.uint8)
+        if _h is None and quality != "realtime":
+            self.set_quality(quality)
 
     def copy(self):
         """Encoder( const Encoder & ) (encoder.cc:92-102): O(1) in pixels, shares the reference rasters"""
@@ -411,11 +414,14 @@ class Encoder:
         return Encoder(self.ctx, _h=h)
 
     @staticmethod
-    def from_decoder(ctx, decoder):
+    def from_decoder(ctx, decoder, quality="realtime"):
         """Encoder( const Decoder &, two_pass, quality ) (encoder.hh:350-351)"""
         h = C.c_void_p()
         check(ctx.L.vp8gpu_encoder_create_from_decoder(ctx.h, decoder.h, C.byref(h)), ctx.h, "encoder_create_from_decoder")
-        return Encoder(ctx, _h=h)
+        enc = Encoder(ctx, _h=h)
+        if quality != "realtime":
+            enc.set_quality(quality)
+        return enc
 
     def export_decoder(self):
         """Encoder::export_decoder (encoder.hh:378)"""
@@ -426,6 +432,15 @@ class Encoder:
     def set_two_pass(self, on):
         """Encoder( ..., two_pass, ... ): key frames get the trellis pass (encoder.cc:220-408)"""
         check(self.L.vp8gpu_encoder_set_two_pass(self.h, int(bool(on))), self.ctx.h, "encoder_set_two_pass")
+
+    def set_quality(self, quality):
+        """Encoder( ..., quality ) (encoder.hh:56-60): "best" tries B_PRED and searches a new motion vector at every
+        inter-frame macroblock and starts every quantiser and loop-filter search from scratch; "realtime" does
+        neither.  LogicError once the encoder has written a frame."""
+        codes = {"best": capi.QUALITY_BEST, "realtime": capi.QUALITY_REALTIME}
+        if quality not in codes:
+            raise capi.LogicError(capi.ERR_LOGIC, "set_quality: %r is neither 'best' nor 'realtime'" % (quality,))
+        check(self.L.vp8gpu_encoder_set_quality(self.h, codes[quality]), self.ctx.h, "encoder_set_quality")
 
     def set_writer(self, mode):
         """0: bitstream byte-identical to the reference encoder's (default); 1: compact writer, 8 partitions"""

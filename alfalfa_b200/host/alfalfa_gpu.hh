@@ -259,6 +259,9 @@ struct SourceFrame {
   size_t y_stride, uv_stride;
 };
 
+// EncoderQuality (encoder/encoder.hh:56-60), same order
+enum EncoderQuality { BEST_QUALITY = VP8GPU_QUALITY_BEST, REALTIME_QUALITY = VP8GPU_QUALITY_REALTIME };
+
 class Encoder {
   Context ctx_;
   uint16_t width_, height_;
@@ -277,6 +280,17 @@ class Encoder {
       : ctx_(decoder.context()), width_(decoder.get_width()), height_(decoder.get_height()),
         buf_(size_t(width_) * height_ * 3 + 65536) {
     check(vp8gpu_encoder_create_from_decoder(ctx_.get(), decoder.handle(), &h_), ctx_.get(), "encoder_create_from_decoder");
+  }
+  // Encoder( width, height, two_pass, quality ) (encoder.hh:346-348)
+  Encoder(const Context& ctx, uint16_t width, uint16_t height, bool two_pass, EncoderQuality quality)
+      : Encoder(ctx, width, height) {
+    set_two_pass(two_pass);
+    set_quality(quality);
+  }
+  // Encoder( const Decoder &, two_pass, quality ) (encoder.hh:350-351)
+  Encoder(const Decoder& decoder, bool two_pass, EncoderQuality quality) : Encoder(decoder) {
+    set_two_pass(two_pass);
+    set_quality(quality);
   }
   // Encoder( const Encoder & ) (encoder.cc:92-102)
   Encoder(const Encoder& o) : ctx_(o.ctx_), width_(o.width_), height_(o.height_), buf_(o.buf_.size()) {
@@ -301,6 +315,8 @@ class Encoder {
   }
   // Encoder( ..., two_pass, ... ) (encoder.hh:347-351): key frames get the trellis pass (encoder.cc:220-408)
   void set_two_pass(bool on) { check(vp8gpu_encoder_set_two_pass(h_, on), ctx_.get(), "set_two_pass"); }
+  // Encoder( ..., quality ): only before the first frame is written (LogicError after)
+  void set_quality(EncoderQuality quality) { check(vp8gpu_encoder_set_quality(h_, quality), ctx_.get(), "set_quality"); }
   // minihash (encoder.hh:382)
   uint32_t minihash() const {
     uint32_t m = 0;

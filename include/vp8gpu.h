@@ -422,6 +422,17 @@ int vp8gpu_encoder_set_writer(vp8gpu_encoder* enc, int mode);
  * with trellis quantisation (Encoder::trellis_quantize, check_reset_y2, encoder/encoder.cc:198-408) priced by the token
  * costs of the default tables; inter frames are coded once either way, as in the reference. */
 int vp8gpu_encoder_set_two_pass(vp8gpu_encoder* enc, int on);
+/* Encoder( ..., quality ) (encoder/encoder.hh:56-60, 346-351), in the reference enum's order.  REALTIME (the default) is
+ * Salsify's setting: inter frames never try B_PRED, NEWMV is searched at every fourth macroblock column and row, and
+ * every frame remembers its quantiser and loop-filter level to narrow the next frame's searches (encoder.cc:164-167).
+ * BEST is ExCamera's xc-enc default: inter frames try B_PRED at every macroblock, NEWMV is searched everywhere, and
+ * nothing is remembered -- every target-size search bisects over [4, 127], every loop-filter search walks up from 0.
+ * It applies to every encode_*, estimate and re-encoding call; the emitted frames are byte-identical to the reference
+ * encoder's at the same setting.  Valid until the encoder writes its first frame (a clone inherits the setting and
+ * whether it may still change); VP8GPU_ERR_LOGIC after that and for other values. */
+#define VP8GPU_QUALITY_BEST     0
+#define VP8GPU_QUALITY_REALTIME 1
+int vp8gpu_encoder_set_quality(vp8gpu_encoder* enc, int quality);
 /* Encoder::encode_with_quantizer (encoder.cc:559-590) */
 int vp8gpu_encoder_encode_with_quantizer(vp8gpu_encoder* enc, const uint8_t* y, size_t y_stride, const uint8_t* u,
                                          const uint8_t* v, size_t uv_stride, int y_ac_qi, uint8_t* out, size_t cap,
@@ -479,7 +490,7 @@ int vp8gpu_encoder_write_frame(vp8gpu_encoder* enc, const vp8gpu_parsed* frame, 
  * quantisers of neighbouring prediction frames, reencode.cc:334-361); -1 without kept labels */
 int vp8gpu_parsed_y_ac_qi(const vp8gpu_parsed* p);
 
-/* EncoderStats (encoder.hh:118-127) of the last frame; any pointer may be NULL. */
+/* EncoderStats (encoder.hh:118-127) of the last frame, at either quality; any pointer may be NULL. */
 int vp8gpu_encoder_stats(const vp8gpu_encoder* enc, double* ssim, int* loop_filter_level, int* y_ac_qi);
 /* Diagnostic: where the host spent the last encode_with_quantizer / encode_with_target_size call, wall-clock
  * milliseconds per phase (each phase ends with the device work it queued being finished, so device time is inside):
